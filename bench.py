@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the B200 MSM / batch-verify engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload msm|verify] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload msm|verify] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): Pippenger MSM points/sec (default workload) and Ed25519 verify_batch
 signatures/sec (reported in the same line under "verify_batch", or as the main metric with
@@ -47,6 +47,21 @@ def dist_env():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     return rank, world, local
+
+
+DUMP_MAX_VALUES = 1 << 21           # per array: 16 MB of float64; larger outputs are sampled at fixed, seeded indices
+
+
+def dump_outputs(path, outputs):
+    """Write each output (bytes: one value per byte; a verdict list or array: one value per entry) as
+    path/<name>.npy in float64, so that two builds run with the same arguments can be compared value for value."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in outputs.items():
+        a = np.frombuffer(v, dtype=np.uint8) if isinstance(v, bytes) else np.atleast_1d(np.asarray(v))
+        if a.size > DUMP_MAX_VALUES:
+            a = a[np.sort(np.random.Generator(np.random.PCG64(SEED)).choice(a.size, DUMP_MAX_VALUES, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
 
 
 def measured_peaks():
@@ -169,7 +184,7 @@ class MsmWorkload:
         return comp
 
 
-def run_msm(args, rank, world, local):
+def run_msm(args, rank, world, local, outputs=None):
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -229,7 +244,7 @@ def run_msm(args, rank, world, local):
     t0 = time.perf_counter()
     call_ms = []
     for _ in range(args.steps):
-        step()
+        comp = step()
         kernel_ms.append(eng.last_kernel_ms()[0])
         call_ms.append(eng.last_call_ms())           # CUDA events on the engine's stream around the MSM call
     barrier()
@@ -247,10 +262,12 @@ def run_msm(args, rank, world, local):
     e0 = time.perf_counter()
     e2e_call_ms = []
     for _ in range(args.steps):
-        step(host=True)
+        comp_e2e = step(host=True)
         e2e_call_ms.append(eng.last_call_ms())
     barrier()
     e1 = time.perf_counter()
+    if outputs is not None:
+        outputs.update(msm_point=comp, msm_point_e2e=comp_e2e)
     clocks = sampler.stop() if rank == 0 else None        # sampled over both timed regions
     e2e_t = torch.tensor([e1 - e0], dtype=torch.float64, device=dev)
     if world > 1:
@@ -404,7 +421,8 @@ def build_verify_inputs(eng, n, nkeys=1024):
     return flat, offs, np.frombuffer(sigs, dtype=np.uint8).copy(), np.frombuffer(pks, dtype=np.uint8).copy()
 
 
-def run_verify(args, rank, world, local, eng=None, steps=None, warmup=None, nkeys=1024, batch_size=None, each=False, key_points=False):
+def run_verify(args, rank, world, local, eng=None, steps=None, warmup=None, nkeys=1024, batch_size=None, each=False, key_points=False,
+               outputs=None):
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -451,23 +469,24 @@ def run_verify(args, rank, world, local, eng=None, steps=None, warmup=None, nkey
             rc = fn(eng.h, b[0].data_ptr(), b[1].data_ptr(), b[2].data_ptr(), b[3].data_ptr(), n, 0, each_res.ctypes.data)
             if rc != 0:
                 raise SystemExit("bench: verify_each rejected valid signatures (rc=%d)" % rc)
-            return
+            return each_res
         if batch_size and key_points:
             rc, verdicts = eng.verify_batches_flat_points(b[0].data_ptr(), b[1].data_ptr(), b[2].data_ptr(), b[3].data_ptr(),
                                                           (hk if host else dk).data_ptr(), n, batch_size, device_ptrs=not host)
             if rc != 0 or any(verdicts):
                 raise SystemExit("bench: verify_batches (key points) rejected valid signatures")
-            return
+            return verdicts
         if batch_size:      # SURVEY 8d config 3B: independent batches of `batch_size`, one verdict each
             rc, verdicts = eng.verify_batches_flat(b[0].data_ptr(), b[1].data_ptr(), b[2].data_ptr(), b[3].data_ptr(), n, batch_size,
                                                    device_ptrs=not host)
             if rc != 0 or any(verdicts):
                 raise SystemExit("bench: verify_batches rejected valid signatures")
-            return
+            return verdicts
         rc = eng.verify_batch_flat(b[0].data_ptr(), b[1].data_ptr(), b[2].data_ptr(), b[3].data_ptr(), n,
                                    device_ptrs=not host, msgs_bytes=n * 59)
         if rc != 0:
             raise SystemExit("bench: verify_batch returned %d on valid signatures" % rc)
+        return rc
 
     def barrier():
         torch.cuda.synchronize()
@@ -502,13 +521,15 @@ def run_verify(args, rank, world, local, eng=None, steps=None, warmup=None, nkey
     t0 = time.perf_counter()
     call_ms, e2e_call_ms, prep_ms = [], [], []
     for _ in range(steps):
-        step()
+        res = step()
         kernel_ms.append(eng.last_kernel_ms()[0])
         call_ms.append(eng.last_call_ms())
         if not each:
             prep_ms.append(eng.last_stage_ms("decompress_R"))
     barrier()
     t1 = time.perf_counter()
+    if outputs is not None:
+        outputs["verify_result"] = np.array(res)          # a copy: verify_each reuses its result buffer in the next loop
     launches = eng.launch_count() - l0
     el = torch.tensor([t1 - t0], dtype=torch.float64, device=dev)
     if world > 1:
@@ -518,10 +539,12 @@ def run_verify(args, rank, world, local, eng=None, steps=None, warmup=None, nkey
     barrier()
     e0 = time.perf_counter()
     for _ in range(steps):
-        step(host=True)
+        res = step(host=True)
         e2e_call_ms.append(eng.last_call_ms())
     barrier()
     e1 = time.perf_counter()
+    if outputs is not None:
+        outputs["verify_result_e2e"] = np.array(res)
     clocks = sampler.stop() if rank == 0 else None
     et = torch.tensor([e1 - e0], dtype=torch.float64, device=dev)
     if world > 1:
@@ -981,9 +1004,14 @@ def main():
     ap.add_argument("--transcript-chunk", type=int, default=64, help="signatures per Merlin transcript in the single-call verify_batch leg (0 = the reference's single transcript)")
     ap.add_argument("--exact-transcript-leg", type=int, default=1, help="also time ONE 2^18-signature verify_batch call with the reference's single transcript")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary verify_batch / cpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed calls returned in their last step (device-resident and from host buffers) "
+                         "as DIR/<name>.npy, float64")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank, world, local = dist_env()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the engine's results: it needs --impl b200")
     if args.impl == "reference":
         line = run_reference(args, rank, world)
         if line is not None:
@@ -995,10 +1023,11 @@ def main():
     import torch.distributed as dist
     if not torch.cuda.is_available():
         raise SystemExit("bench: no CUDA device; the engine has no CPU fallback")
+    outputs = {}
     if args.workload == "verify":
-        line = run_verify(args, rank, world, local)
+        line = run_verify(args, rank, world, local, outputs=outputs)
     else:
-        line, eng, wl = run_msm(args, rank, world, local)
+        line, eng, wl = run_msm(args, rank, world, local, outputs=outputs)
         if not args.no_extras and world > 1:
             # BASELINE.json's metric names verify_batch at 1/2/4/8 GPUs too: independent replicas, one batch per GPU
             v = run_verify(args, rank, world, local, eng=eng, steps=min(args.steps, 5), warmup=3)
@@ -1058,6 +1087,8 @@ def main():
                 v2, dt2 = cpu_verify_baseline(4096, 1)
                 line["verify_batch"]["cpu_baseline"] = {"value": v2, "unit": "sigs/s", "cores": 1, "kind": "port",
                                                         "sample": "16 oracle verify_batch calls of 256 signatures, 1 thread (%.1f s)" % dt2}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1 and dist.is_initialized():

@@ -1,7 +1,8 @@
 """One pass over the widened rows (SURVEY 8f) for profiling: batch codecs on 2^20 points, per-signature verification on
 2^20 signatures, precomputed MSM over 2^20 resident points."""
-import sys, ctypes as C
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, ctypes as C
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import curve25519_dalek_b200 as pkg
 import bench

@@ -1,7 +1,8 @@
 """Time the Ristretto double-base batch (BASELINE configs[4]) through the per-pair Straus kernel (0) and the
 fixed-base comb kernel (1); checksums must agree."""
-import sys
-sys.path.insert(0, "/root/repo")
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import curve25519_dalek_b200 as pkg
 import bench
 eng = pkg.Engine(0)

@@ -1,6 +1,7 @@
 """Precomputed MSM over 2^20 resident points: window tables on/off x scalar chunks, wall / device / accumulate ms."""
-import sys, time, ctypes as C
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, time, ctypes as C
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import curve25519_dalek_b200 as pkg
 import bench

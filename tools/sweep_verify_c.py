@@ -1,5 +1,6 @@
-import sys, time
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, time
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import curve25519_dalek_b200 as pkg
 import bench

@@ -1,7 +1,8 @@
 """Per-stage device timeline (option "trace") of verify calls over 2^22 signatures: independent batches of 256, device-resident
 and from pinned host buffers (pieces streamed over PCIe), for 1..8 pieces.  Run on the B200; the timeline goes to stderr."""
-import sys
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 torch.set_num_threads(1)            # pinned buffers first-touched by one thread (NUMA-local): 55 instead of 35 GB/s over PCIe
 import curve25519_dalek_b200 as pkg
