@@ -59,7 +59,8 @@ void dalek_b200_destroy(dalek_b200_ctx *ctx)
     DevBuf *bufs[] = {&ctx->scalars, &ctx->points_in, &ctx->points, &ctx->digits, &ctx->counts, &ctx->offsets,
                       &ctx->sorted, &ctx->buckets, &ctx->red_a, &ctx->red_b, &ctx->red_c, &ctx->red_d, &ctx->key_pts,
                       &ctx->result, &ctx->flags, &ctx->misc0, &ctx->misc1, &ctx->misc2, &ctx->misc3,
-                      &ctx->misc4, &ctx->misc5, &ctx->zs, &ctx->base_table, &ctx->ntasks, &ctx->task_off, &ctx->tasks, &ctx->task_sums, &ctx->msg_offs, &ctx->sum_desc, &ctx->sum_part, &ctx->key_table, &ctx->key_acc, &ctx->task_order, &ctx->sig_status, &ctx->misc6, &ctx->each_pow, &ctx->each_tab, &ctx->each_kstat};
+                      &ctx->misc4, &ctx->misc5, &ctx->zs, &ctx->base_table, &ctx->ntasks, &ctx->task_off, &ctx->tasks, &ctx->task_sums, &ctx->msg_offs, &ctx->sum_desc, &ctx->sum_part, &ctx->key_table, &ctx->key_acc, &ctx->task_order, &ctx->sig_status, &ctx->misc6, &ctx->each_pow, &ctx->each_tab, &ctx->each_kstat,
+                      &ctx->bt_meta, &ctx->bt_status, &ctx->bt_res, &ctx->bt_nafs, &ctx->bt_tables, &ctx->bt_part};
     for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
     cudaEventDestroy(ctx->ev_a); cudaEventDestroy(ctx->ev_b); cudaEventDestroy(ctx->ev_fork); cudaEventDestroy(ctx->ev_join);
@@ -88,6 +89,7 @@ int dalek_b200_set_option(dalek_b200_ctx *ctx, const char *name, long value)
     if (!strcmp(name, "each_comb")) { if (value < 0 || value > 2) return DALEK_E_INVALID_ARG; ctx->opt_each_comb = value; return 0; }
     if (!strcmp(name, "small_straus")) { ctx->opt_small_straus = value ? 1 : 0; return 0; }
     if (!strcmp(name, "acc_tma")) { ctx->opt_acc_tma = value ? 1 : 0; return 0; }
+    if (!strcmp(name, "batch_bucket_min")) { if (value < 1 || value > 0x7fffffffL) return DALEK_E_INVALID_ARG; ctx->opt_batch_bucket_min = value; return 0; }
     if (!strcmp(name, "field_f64")) { ctx->opt_field_f64 = value ? 1 : 0; return 0; }
     if (!strcmp(name, "verify_chunk")) { if (value < 0 || value > (1 << 20)) return DALEK_E_INVALID_ARG; ctx->opt_verify_chunk = value; return 0; }
     return DALEK_E_INVALID_ARG;

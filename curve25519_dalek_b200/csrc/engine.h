@@ -11,6 +11,10 @@
 
 #include "ge.cuh"
 
+// Batched MSM: default of the option "batch_bucket_min" (msm_batch.cu): the best value of the sweep in
+// tools/msm_batch_bench.py on a B200 (profiles/msm_batch_r1.json)
+#define BATCH_BUCKET_MIN_DEFAULT 65536
+
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
@@ -49,6 +53,7 @@ struct dalek_b200_ctx {
     long opt_each_comb = 1;     // verify_each: 1 = per-key comb tables when every key signs >= 8 signatures on average, 2 = always, 0 = never
     long opt_small_straus = 1;  // fewer than 190 pairs: vartime Straus (3 launches) instead of the bucket pipeline
     long opt_field_f64 = 1;     // bucket kernel on the FP64 pipe (fe64.cuh) instead of IMAD.WIDE (fe.cuh)
+    long opt_batch_bucket_min = BATCH_BUCKET_MIN_DEFAULT;   // batched MSM: segments of at least this many pairs take the bucket pipeline
     // timing of the dominant kernel in the last call
     float last_kernel_ms = 0.f;
     float last_call_ms = 0.f;
@@ -56,7 +61,8 @@ struct dalek_b200_ctx {
     bool async_open = false;       // a ..._partial_async call is in flight: its device span ends in ..._combine_dev
     // device workspaces (grown on demand, reused across calls)
     DevBuf scalars, points_in, points, digits, counts, offsets, sorted, buckets, red_a, red_b, red_c,
-        red_d, key_pts, result, flags, misc0, misc1, misc2, misc3, misc4, misc5, zs, base_table, ntasks, task_off, tasks, task_sums, msg_offs, sum_desc, sum_part, key_table, key_acc, task_order, sig_status, misc6, each_pow, each_tab, each_kstat;
+        red_d, key_pts, result, flags, misc0, misc1, misc2, misc3, misc4, misc5, zs, base_table, ntasks, task_off, tasks, task_sums, msg_offs, sum_desc, sum_part, key_table, key_acc, task_order, sig_status, misc6, each_pow, each_tab, each_kstat,
+        bt_meta, bt_status, bt_res, bt_nafs, bt_tables, bt_part;   // batched MSM (msm_batch.cu)
     const uint64_t *key_points = nullptr;   // device: callers' decompressed key points for the current verify_batch call (or null)
     uint32_t hash_seed[4] = {0x243F6A88u, 0x85A308D3u, 0x13198A2Eu, 0x03707344u};   // key of the public-key de-duplication hash, redrawn per context
     int sum_desc_c = -1;
@@ -190,6 +196,29 @@ int straus_ct_msm(dalek_b200_ctx *ctx, const uint32_t *d_scalars, const void *d_
 int base_table_ensure(dalek_b200_ctx *ctx);
 
 int ristretto_prepare_points(dalek_b200_ctx *ctx, const void *d_in, size_t n, void *d_out, int *d_bad);
+
+// ---- batched MSM (msm_batch.cu): building blocks in msm.cu / straus.cu / straus_vt.cu ----
+// A point that does not decode marks its SEGMENT: bad[k] = 1 for the k with offs[k] <= base + i < offs[k + 1]
+// (offs: m + 1 non-decreasing device u64), instead of the call-wide flag.
+struct SegStatus { const uint64_t *offs; size_t m; uint64_t base; uint32_t *bad; };
+#ifdef __CUDACC__
+__device__ __forceinline__ void seg_mark_bad(const SegStatus &s, size_t i)
+{
+    const uint64_t g = s.base + i;
+    size_t lo = 0, hi = s.m;                       // last k with offs[k] <= g (empty segments are skipped)
+    while (hi - lo > 1) { const size_t mid = (lo + hi) / 2; if (s.offs[mid] <= g) lo = mid; else hi = mid; }
+    s.bad[lo] = 1;
+}
+#endif
+// point_fmt: DALEK_POINTS_COMPRESSED (-> PK_NIELS), _EXTENDED or _RISTRETTO (-> PK_PNIELS)
+int msm_prepare_points_seg(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in, int point_fmt, size_t n, void *d_out,
+                           const SegStatus &seg);
+int ristretto_prepare_points_seg(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in, size_t n, void *d_out, const SegStatus &seg);
+// width-5 NAF (NAF_LEN bytes) and the table of odd multiples (8 projective Niels) of n pairs (k_straus_prepare)
+int straus_prepare(dalek_b200_ctx *ctx, cudaStream_t st, const uint32_t *d_scalars, const void *d_points, int point_kind, size_t n,
+                   int8_t *d_nafs, ge_pniels_packed *d_tables);
+// out[k] = sum of pool[d.x .. d.x + d.y) for the count descriptors d = desc[k] (uint2, device)
+int msm_plain_sums(dalek_b200_ctx *ctx, cudaStream_t st, const ge_p3_raw *pool, const void *d_desc, uint32_t count, ge_p3_raw *out);
 int ristretto_encode_result(dalek_b200_ctx *ctx, const MsmResult *d_res, uint32_t *d_enc);
 int ristretto_double_base(dalek_b200_ctx *ctx, const uint8_t *d_a, const uint8_t *d_b, const uint8_t G[32],
                           const uint8_t H[32], size_t n, uint8_t *d_out, int *h_status);

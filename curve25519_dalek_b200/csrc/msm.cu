@@ -62,9 +62,10 @@ int pinned_reserve(dalek_b200_ctx *ctx, size_t bytes)
 
 // ------------------------------------------------------------------------------------------
 // point preparation
-template <int F64>
+// SEG = 1: a point that does not decode marks its segment (batched MSM) instead of the call-wide flag
+template <int F64, int SEG>
 __global__ void __launch_bounds__(128, 3) k_prep_compressed(const uint4 *__restrict__ in, ge_niels_packed *__restrict__ out, size_t n,
-                                  int *__restrict__ bad)
+                                  int *__restrict__ bad, SegStatus seg)
 {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -72,7 +73,10 @@ __global__ void __launch_bounds__(128, 3) k_prep_compressed(const uint4 *__restr
     uint32_t s[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
     fe x, y;
     uint32_t ok = ge_decompress_affine<F64>(x, y, s);
-    if (!ok) { atomicOr(bad, 1); fe_0(x); fe_1(y); }   // identity placeholder keeps the kernels total
+    if (!ok) {                                          // identity placeholder keeps the kernels total
+        if (SEG) seg_mark_bad(seg, i); else atomicOr(bad, 1);
+        fe_0(x); fe_1(y);
+    }
     ge_niels nl; ge_affine_to_niels(nl, x, y);
     ge_niels_packed p; ge_niels_pack(p, nl);
     uint4 *o = reinterpret_cast<uint4 *>(out + i);
@@ -101,8 +105,8 @@ int msm_prepare_points_on(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in
 {
     if (n == 0) return 0;
     if (point_fmt == DALEK_POINTS_COMPRESSED) {
-        if (ctx->opt_decompress_f64) k_prep_compressed<1><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, d_bad);
-        else k_prep_compressed<0><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, d_bad);
+        if (ctx->opt_decompress_f64) k_prep_compressed<1, 0><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, d_bad, SegStatus{});
+        else k_prep_compressed<0, 0><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, d_bad, SegStatus{});
     } else {
         k_prep_extended<<<cdiv(n, 128), 128, 0, st>>>((const uint64_t *)d_in, (ge_pniels_packed *)d_out, n);
     }
@@ -114,6 +118,22 @@ int msm_prepare_points_on(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in
 int msm_prepare_points(dalek_b200_ctx *ctx, const void *d_in, int point_fmt, size_t n, void *d_out, int *d_bad)
 {
     return msm_prepare_points_on(ctx, ctx->stream, d_in, point_fmt, n, d_out, d_bad);
+}
+
+int msm_prepare_points_seg(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in, int point_fmt, size_t n, void *d_out,
+                           const SegStatus &seg)
+{
+    if (n == 0) return 0;
+    if (point_fmt == DALEK_POINTS_RISTRETTO) return ristretto_prepare_points_seg(ctx, st, d_in, n, d_out, seg);
+    if (point_fmt == DALEK_POINTS_COMPRESSED) {
+        if (ctx->opt_decompress_f64) k_prep_compressed<1, 1><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, nullptr, seg);
+        else k_prep_compressed<0, 1><<<cdiv(n, 128), 128, 0, st>>>((const uint4 *)d_in, (ge_niels_packed *)d_out, n, nullptr, seg);
+    } else {
+        k_prep_extended<<<cdiv(n, 128), 128, 0, st>>>((const uint64_t *)d_in, (ge_pniels_packed *)d_out, n);
+    }
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -660,6 +680,15 @@ k_plain_sum(const ge_p3_raw *__restrict__ pool, const uint2 *__restrict__ desc, 
         __syncthreads();
     }
     if (grp == 0) { w4_load(acc, &sh[0]); w4_store(out + blockIdx.x, acc, role); }
+}
+
+int msm_plain_sums(dalek_b200_ctx *ctx, cudaStream_t st, const ge_p3_raw *pool, const void *d_desc, uint32_t count, ge_p3_raw *out)
+{
+    if (!count) return 0;
+    k_plain_sum<<<count, 128, 0, st>>>(pool, (const uint2 *)d_desc, out);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
 }
 
 // per window: target = A_1 + m_1 (A_2 + m_2 (...)); A sums are laid out [level][window]

@@ -385,8 +385,10 @@ int ristretto_double_base(dalek_b200_ctx *ctx, const uint8_t *d_a, const uint8_t
 // ------------------------------------------------------------------------------------------
 // Ristretto vartime MSM: decode with the Ristretto rules, then the Edwards bucket MSM; encode the
 // result with RistrettoPoint::compress (ristretto.rs:980-994).
-template <int F64>
-__global__ void k_prep_ristretto(const uint32_t *__restrict__ in, ge_pniels_packed *__restrict__ out, size_t n, int *__restrict__ bad)
+// SEG = 1: a point that does not decode marks its segment (batched MSM) instead of the call-wide flag
+template <int F64, int SEG>
+__global__ void k_prep_ristretto(const uint32_t *__restrict__ in, ge_pniels_packed *__restrict__ out, size_t n, int *__restrict__ bad,
+                                 SegStatus seg)
 {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -394,7 +396,10 @@ __global__ void k_prep_ristretto(const uint32_t *__restrict__ in, ge_pniels_pack
 #pragma unroll
     for (int k = 0; k < 8; k++) enc[k] = in[8 * i + k];
     ge_p3 P;
-    if (!ristretto_decompress<F64>(P, enc)) { atomicOr(bad, 1); ge_p3_identity(P); }
+    if (!ristretto_decompress<F64>(P, enc)) {
+        if (SEG) seg_mark_bad(seg, i); else atomicOr(bad, 1);
+        ge_p3_identity(P);
+    }
     ge_pniels pn; ge_p3_to_pniels(pn, P);
     ge_pniels_packed pk; ge_pniels_pack(pk, pn);
     out[i] = pk;
@@ -414,8 +419,18 @@ __global__ void k_ristretto_encode_result(const MsmResult *__restrict__ res, uin
 int ristretto_prepare_points(dalek_b200_ctx *ctx, const void *d_in, size_t n, void *d_out, int *d_bad)
 {
     if (!n) return 0;
-    if (ctx->opt_decompress_f64) k_prep_ristretto<1><<<cdiv(n, 128), 128, 0, ctx->stream>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, d_bad);
-    else k_prep_ristretto<0><<<cdiv(n, 128), 128, 0, ctx->stream>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, d_bad);
+    if (ctx->opt_decompress_f64) k_prep_ristretto<1, 0><<<cdiv(n, 128), 128, 0, ctx->stream>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, d_bad, SegStatus{});
+    else k_prep_ristretto<0, 0><<<cdiv(n, 128), 128, 0, ctx->stream>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, d_bad, SegStatus{});
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+
+int ristretto_prepare_points_seg(dalek_b200_ctx *ctx, cudaStream_t st, const void *d_in, size_t n, void *d_out, const SegStatus &seg)
+{
+    if (!n) return 0;
+    if (ctx->opt_decompress_f64) k_prep_ristretto<1, 1><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, nullptr, seg);
+    else k_prep_ristretto<0, 1><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)d_in, (ge_pniels_packed *)d_out, n, nullptr, seg);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
     return 0;
@@ -538,8 +553,8 @@ int dalek_b200_ristretto_vartime_msm(dalek_b200_ctx *ctx, const uint8_t *scalars
     if (n) {
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->scalars.p, scalars, n * 32, cudaMemcpyHostToDevice, st));
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->points_in.p, points, n * 32, cudaMemcpyHostToDevice, st));
-        if (ctx->opt_decompress_f64) k_prep_ristretto<1><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)ctx->points_in.p, (ge_pniels_packed *)ctx->points.p, n, (int *)ctx->flags.p);
-        else k_prep_ristretto<0><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)ctx->points_in.p, (ge_pniels_packed *)ctx->points.p, n, (int *)ctx->flags.p);
+        if (ctx->opt_decompress_f64) k_prep_ristretto<1, 0><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)ctx->points_in.p, (ge_pniels_packed *)ctx->points.p, n, (int *)ctx->flags.p, SegStatus{});
+        else k_prep_ristretto<0, 0><<<cdiv(n, 128), 128, 0, st>>>((const uint32_t *)ctx->points_in.p, (ge_pniels_packed *)ctx->points.p, n, (int *)ctx->flags.p, SegStatus{});
         ctx->launches++;
     }
     int c = msm_choose_window_bits(ctx, n);

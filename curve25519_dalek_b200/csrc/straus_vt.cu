@@ -68,6 +68,18 @@ k_straus_vartime(const int8_t *__restrict__ nafs, const ge_pniels_packed *__rest
     }
 }
 
+int straus_prepare(dalek_b200_ctx *ctx, cudaStream_t st, const uint32_t *d_scalars, const void *d_points, int point_kind, size_t n,
+                   int8_t *d_nafs, ge_pniels_packed *d_tables)
+{
+    if (!n) return 0;
+    const unsigned grid = (unsigned)((n + 63) / 64);
+    if (point_kind == PK_NIELS) k_straus_prepare<PK_NIELS><<<grid, 64, 0, st>>>(d_scalars, d_points, n, d_nafs, d_tables);
+    else k_straus_prepare<PK_PNIELS><<<grid, 64, 0, st>>>(d_scalars, d_points, n, d_nafs, d_tables);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+
 // sum scalars[i] * points[i] for n < 2^16 prepared points (PK_NIELS / PK_PNIELS); result like msm_full
 int straus_vartime_msm(dalek_b200_ctx *ctx, const uint32_t *d_scalars, const void *d_points, int point_kind, size_t n,
                        MsmResult *d_result)
@@ -80,13 +92,9 @@ int straus_vartime_msm(dalek_b200_ctx *ctx, const uint32_t *d_scalars, const voi
     if ((rc = ws_reserve(ctx, ctx->red_b, (nwarps ? nwarps : 1) * sizeof(ge_p3_raw)))) return rc;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_a, st));             // ev_a .. ev_b: the Straus kernels (also recorded for n = 0)
     if (n) {
-        const unsigned grid = (unsigned)((n + 63) / 64);
-        if (point_kind == PK_NIELS)
-            k_straus_prepare<PK_NIELS><<<grid, 64, 0, st>>>(d_scalars, d_points, n, (int8_t *)ctx->digits.p, (ge_pniels_packed *)ctx->red_a.p);
-        else
-            k_straus_prepare<PK_PNIELS><<<grid, 64, 0, st>>>(d_scalars, d_points, n, (int8_t *)ctx->digits.p, (ge_pniels_packed *)ctx->red_a.p);
+        if ((rc = straus_prepare(ctx, st, d_scalars, d_points, point_kind, n, (int8_t *)ctx->digits.p, (ge_pniels_packed *)ctx->red_a.p))) return rc;
         k_straus_vartime<<<(unsigned)nwarps, 32, 0, st>>>((const int8_t *)ctx->digits.p, (const ge_pniels_packed *)ctx->red_a.p, n, (ge_p3_raw *)ctx->red_b.p);
-        ctx->launches += 2;
+        ctx->launches++;
     }
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_b, st));
     ctx->last_kernel_launches = 1;

@@ -82,7 +82,7 @@ W4_DEV void straus_warp(w4f_point &Q, const int8_t *nafs, const ge_pniels_packed
     for (int i = top; i >= 0; i--) {
         const int d = live ? naf[i] : 0;
         const bool any = w4_any(d != 0);
-        if (i != top) w4f_dbl(Q, role, any);
+        if (i != top) w4f_dbl(Q, role, any || i == 0);             // the sums below read T of the final Q
         if (any) {                                                 // uniform per warp: full-mask shuffles inside
             const uint32_t neg = d < 0, e = (uint32_t)(neg ? -d : d) >> 1;      // window.rs:187-192: entry |x| / 2
             ge_pniels_packed pk;

@@ -140,10 +140,9 @@ W4_DEV void w4f_add(w4f_point &p, const w4f_point &q, const fe64 &d2, uint32_t r
     w4f_add_tail(p, a, b, c, D, 0u, role);
 }
 
-// p <- p + q or p - q for a packed projective Niels point (curve_models.rs:411-452 + :365-372)
-W4_DEV void w4f_padd(w4f_point &p, const ge_pniels_packed &pk, uint32_t neg, uint32_t role)
+// p <- p + q or p - q for a projective Niels point whose coordinates have scale <= 2 (curve_models.rs:411-452 + :365-372)
+W4_DEV void w4f_padd_pn(w4f_point &p, const ge64_pniels &q, uint32_t neg, uint32_t role)
 {
-    ge64_pniels q; ge64_pniels_unpack(q, pk);                 // coordinates in [0, 2^51): scale 2
     fe64 qp = q.YpX, qm = q.YmX;
     { fe64 t = qp; fe64_cmov(qp, qm, neg); fe64_cmov(qm, t, neg); }
     fe64 A, B, f, g, r, a, b, c, zz, D;
@@ -154,6 +153,13 @@ W4_DEV void w4f_padd(w4f_point &p, const ge_pniels_packed &pk, uint32_t neg, uin
     fe64_gbcast(a, r, 0); fe64_gbcast(b, r, 1); fe64_gbcast(c, r, 2); fe64_gbcast(zz, r, 3);
     fe64_add(D, zz, zz);
     w4f_add_tail(p, a, b, c, D, neg, role);
+}
+
+// the same for a packed projective Niels point
+W4_DEV void w4f_padd(w4f_point &p, const ge_pniels_packed &pk, uint32_t neg, uint32_t role)
+{
+    ge64_pniels q; ge64_pniels_unpack(q, pk);                 // coordinates in [0, 2^51): scale 2
+    w4f_padd_pn(p, q, neg, role);
 }
 
 // copy of the point held by the group `delta_lanes` lanes above (delta_lanes a multiple of 4)

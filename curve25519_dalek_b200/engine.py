@@ -39,6 +39,9 @@ def load_library():
     lib.dalek_b200_last_stage_ms.argtypes = [vp, C.c_char_p, C.POINTER(C.c_float)]
     for name in ("dalek_b200_edwards_vartime_msm", "dalek_b200_edwards_ct_msm", "dalek_b200_edwards_vartime_msm_dev"):
         getattr(lib, name).argtypes = [vp, vp, vp, C.c_int, sz, vp, vp]
+    lib.dalek_b200_edwards_vartime_msm_batch.argtypes = [vp, vp, vp, C.c_int, vp, sz, vp, vp, vp]
+    lib.dalek_b200_edwards_vartime_msm_batch_dev.argtypes = [vp, vp, vp, C.c_int, vp, sz, vp, vp, vp]
+    lib.dalek_b200_ristretto_vartime_msm_batch.argtypes = [vp, vp, vp, vp, sz, vp, vp]
     lib.dalek_b200_msm_window_count.argtypes = [vp, sz]
     lib.dalek_b200_edwards_msm_partial.argtypes = [vp, vp, vp, C.c_int, sz, sz, vp]
     lib.dalek_b200_edwards_msm_partial_dev.argtypes = [vp, vp, vp, C.c_int, sz, sz, vp]
@@ -188,6 +191,43 @@ class Engine:
                             C.addressof(limbs) if want_limbs else None))
         del keep
         return rc, bytes(out), (list(limbs) if want_limbs else None)
+
+    @staticmethod
+    def _offsets(offsets):
+        if len(offsets) < 1:
+            raise ValueError("offsets holds m + 1 entries (at least [0])")
+        offs = offsets if isinstance(offsets, C.Array) else (C.c_uint64 * len(offsets))(*[int(o) for o in offsets])
+        return offs, len(offs) - 1
+
+    def edwards_vartime_msm_batch(self, scalars, points, offsets, point_fmt=POINTS_COMPRESSED, device_ptrs=False, want_limbs=False):
+        """m = len(offsets) - 1 independent MSMs in one call: MSM k takes the pairs [offsets[k], offsets[k+1]) of the flat
+        scalars / points buffers (offsets: host, offsets[0] = 0, non-decreasing).  Returns (rc, results, limbs): results[k] is
+        the 32-byte compressed result or None (a point of segment k did not decode), limbs (want_limbs) m lists of 20 u64
+        (canonical limbs of an equal point; zeros for None); rc 1 if any result is None."""
+        offs, m = self._offsets(offsets)
+        out = (C.c_uint8 * (32 * max(m, 1)))()
+        st = (C.c_uint8 * max(m, 1))()
+        limbs = (C.c_uint64 * (20 * max(m, 1)))() if want_limbs else None
+        fn = self.lib.dalek_b200_edwards_vartime_msm_batch_dev if device_ptrs else self.lib.dalek_b200_edwards_vartime_msm_batch
+        keep = (scalars, points)
+        rc = self._check(fn(self.h, _ptr(scalars), _ptr(points), point_fmt, C.addressof(offs), m, C.addressof(out),
+                            C.addressof(limbs) if want_limbs else None, C.addressof(st)))
+        del keep
+        raw = bytes(out)
+        res = [None if st[k] else raw[32 * k:32 * k + 32] for k in range(m)]
+        return rc, res, ([list(limbs[20 * k:20 * k + 20]) for k in range(m)] if want_limbs else None)
+
+    def ristretto_vartime_msm_batch(self, scalars, points, offsets):
+        """The Ristretto form of edwards_vartime_msm_batch (CompressedRistretto points and results): (rc, results)."""
+        offs, m = self._offsets(offsets)
+        out = (C.c_uint8 * (32 * max(m, 1)))()
+        st = (C.c_uint8 * max(m, 1))()
+        keep = (scalars, points)
+        rc = self._check(self.lib.dalek_b200_ristretto_vartime_msm_batch(self.h, _ptr(scalars), _ptr(points), C.addressof(offs), m,
+                                                                         C.addressof(out), C.addressof(st)))
+        del keep
+        raw = bytes(out)
+        return rc, [None if st[k] else raw[32 * k:32 * k + 32] for k in range(m)]
 
     def edwards_ct_msm(self, scalars, points, n, point_fmt=POINTS_COMPRESSED, want_limbs=False):
         out = (C.c_uint8 * 32)()
@@ -434,6 +474,12 @@ class EdwardsPoint:
         return None if rc == 1 else comp
 
     @staticmethod
+    def optional_multiscalar_mul_batch(msms, engine=None):
+        """optional_multiscalar_mul for every (scalars, points) of `msms` in one engine call: a list of Optional[bytes].
+        A point that is None or does not decompress makes that MSM's result None, and only that one."""
+        return _msm_batch(msms, engine, ristretto=False)
+
+    @staticmethod
     def vartime_multiscalar_mul(scalars, points, engine=None):
         """traits.rs:249-262: .expect() on the optional form."""
         r = EdwardsPoint.optional_multiscalar_mul(scalars, points, engine)
@@ -449,6 +495,30 @@ class EdwardsPoint:
         eng = engine or default_engine()
         rc, comp, _ = eng.edwards_ct_msm(b"".join(scalars), b"".join(points), len(scalars))
         return comp
+
+
+# encodings that never decode, standing in for None points: y = 2 is not on the curve; s = 1 is a negative field element,
+# which CompressedRistretto::decompress rejects (ristretto.rs:266-345)
+_BAD_EDWARDS = (2).to_bytes(32, "little")
+_BAD_RISTRETTO = (1).to_bytes(32, "little")
+
+
+def _msm_batch(msms, engine, ristretto):
+    sc, pt, offsets = [], [], [0]
+    bad = _BAD_RISTRETTO if ristretto else _BAD_EDWARDS
+    for scalars, points in msms:
+        scalars, points = list(scalars), list(points)
+        assert len(scalars) == len(points), "scalars and points must have the same length"
+        sc += scalars
+        pt += [bad if p is None else p for p in points]
+        offsets.append(len(sc))
+    eng = engine or default_engine()
+    sb, pb = b"".join(sc), b"".join(pt)
+    if ristretto:
+        _, res = eng.ristretto_vartime_msm_batch(sb, pb, offsets)
+    else:
+        _, res, _ = eng.edwards_vartime_msm_batch(sb, pb, offsets)
+    return res
 
 
 class _Precomputation:
@@ -536,6 +606,12 @@ class RistrettoPoint:
         if rc == 1:
             raise ValueError("should return some point")
         return comp
+
+    @staticmethod
+    def optional_multiscalar_mul_batch(msms, engine=None):
+        """Independent Ristretto MSMs in one engine call (CompressedRistretto points and results): a list of
+        Optional[bytes]; a None or undecodable point makes that MSM's result None, and only that one."""
+        return _msm_batch(msms, engine, ristretto=True)
 
     @staticmethod
     def double_base_batch(a, b, G, H, engine=None):

@@ -71,8 +71,9 @@ const char *dalek_b200_last_error(const dalek_b200_ctx *ctx);
  * kernel what the shorter tail saves), "transcript_warp" (1 = launches of up to 2048 Merlin transcripts run one warp each,
  * default), "transcript_blocks" (1 = larger launches run one thread per transcript with the rate block staged in shared
  * memory, default; 0 = byte-wise sponge), "each_comb" (per-signature verification: 1 = per-key comb tables when
- * every distinct key signs at least eight signatures on average, default; 2 = always; 0 = never), "trace" (1 = per-stage
- * device timeline of verify_batch on stderr).
+ * every distinct key signs at least eight signatures on average, default; 2 = always; 0 = never), "batch_bucket_min"
+ * (1..2^31-1: segments of a batched MSM with at least this many pairs run the bucket pipeline, shorter ones the
+ * segmented Straus; default 65536), "trace" (1 = per-stage device timeline of verify_batch on stderr).
  * Returns 0 or DALEK_E_INVALID_ARG. */
 int dalek_b200_set_option(dalek_b200_ctx *ctx, const char *name, long value);
 /* Number of kernels launched by this context since creation (bench.py's gpu_launches). */
@@ -117,6 +118,31 @@ int dalek_b200_edwards_ct_msm(dalek_b200_ctx *ctx, const uint8_t *scalars, const
 int dalek_b200_edwards_vartime_msm_dev(dalek_b200_ctx *ctx, const void *d_scalars, const void *d_points,
                                        int point_fmt, size_t n, uint8_t out_compressed[32],
                                        uint64_t out_limbs[20]);
+
+/* -------- many independent MSMs in one call ------------------------------------------------
+ * m independent VartimeMultiscalarMul::optional_multiscalar_mul calls (C/traits.rs:196-262) in one call.
+ * MSM k takes the pairs [offsets[k], offsets[k+1]) of the flat scalars / points arrays (offsets: m + 1 u64, HOST memory
+ * in both forms, offsets[0] = 0, non-decreasing, offsets[m] < 2^31).  Result k is byte for byte what
+ * dalek_b200_edwards_vartime_msm returns on slice k: out_compressed[32 k ..] the CompressedEdwardsY, out_limbs[20 k ..]
+ * (nullable) canonical limbs of an equal point, status[k] = 1 (None) when a point of segment k does not decode -- its 32
+ * output bytes (and limbs) are then zero; a bad point affects only its own segment.  point_fmt: COMPRESSED or EXTENDED;
+ * scalars may be any 256-bit value; an empty segment gives the identity with status 0.
+ * Returns 0 if every status is 0, DALEK_NONE if any is 1, DALEK_E_INVALID_ARG for malformed offsets, null buffers or a bad
+ * point_fmt, or m >= 2^31, other negative codes for engine errors; m = 0 succeeds and writes nothing.  dalek_b200_last_call_ms covers
+ * the whole call.  Segments shorter than the option "batch_bucket_min" (default 65536 pairs) run as a segmented Straus
+ * (one accumulator per task of up to 64 pairs of one segment), all of them in a few launches per ~2^20 pairs; longer
+ * segments, and any longer than 2^20 pairs, run the bucket pipeline one after another.  The results do not depend on the
+ * option. */
+int dalek_b200_edwards_vartime_msm_batch(dalek_b200_ctx *ctx, const uint8_t *scalars, const void *points, int point_fmt,
+                                         const uint64_t *offsets, size_t m, uint8_t *out_compressed /* m x 32 */,
+                                         uint64_t *out_limbs /* nullable, m x 20 */, uint8_t *status /* m */);
+/* The same with device-resident scalars and points; offsets and outputs are host memory. */
+int dalek_b200_edwards_vartime_msm_batch_dev(dalek_b200_ctx *ctx, const void *d_scalars, const void *d_points, int point_fmt,
+                                             const uint64_t *offsets, size_t m, uint8_t *out_compressed,
+                                             uint64_t *out_limbs, uint8_t *status);
+/* RistrettoPoint form over CompressedRistretto points; result k as dalek_b200_ristretto_vartime_msm returns it on slice k. */
+int dalek_b200_ristretto_vartime_msm_batch(dalek_b200_ctx *ctx, const uint8_t *scalars, const uint8_t *points,
+                                           const uint64_t *offsets, size_t m, uint8_t *out_compressed, uint8_t *status);
 
 /* -------- sharded MSM (one call per GPU / rank, SURVEY 8e) --------------------------------
  * MSM is linear: every rank reduces a contiguous shard of the pairs to one accumulator per bucket window
